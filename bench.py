@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --steps K --warmup W    # the reference algorithm on the host CPU (oracle port)
+  python bench.py --steps K --warmup W --dump-outputs DIR  # + the last timed step's outputs as DIR/<name>.npy
 
 One step = one loop body of generate_samples_from_batch (reference model_v2w.py:130-149): sampler glue +
 cond forward + uncond forward of the 28-block 7B DiT over the 121-frame / 704x1280 latent [16,16,88,160]
@@ -30,12 +31,29 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 FLOP_PER_FORWARD = 2.2096e15  # SURVEY.md §8d / BASELINE.md §2
 FLOP_PER_STEP = 2 * FLOP_PER_FORWARD
 SELF_ATTN_FLOP_PER_LAUNCH_FULL = 4.0 * 56320 * 56320 * 4096  # 5.197e13 at cp = 1
 LAT = (16, 16, 88, 160)
 CTX = (512, 1024)
+DUMP_SAMPLE = 1 << 20  # elements kept of each Path R output (1.7 GB per render) by --dump-outputs
+
+
+def seeded_sample(torch, t):
+    """The same DUMP_SAMPLE elements of any tensor of t's size, so that two builds can be compared output for output."""
+    idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0))
+    return t.reshape(-1)[idx.to(t.device)]
+
+
+def dump_outputs(dump_dir, outputs):
+    """Writes each tensor as dump_dir/<name>.npy in float32."""
+    import numpy as np
+
+    os.makedirs(dump_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(dump_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def measured_peaks():
@@ -193,7 +211,8 @@ def path_r_cpu_frames_per_s(n_frames: int = 4):
     return n_frames / dt, dt, 1
 
 
-def bench_path_r(torch, dev, peaks, steps: int, warmup: int, cpu_baseline: bool):
+def bench_path_r(torch, dev, peaks, steps: int, warmup: int, cpu_baseline: bool, outputs=None):
+    """outputs: dict that receives a seeded sample of the pixels and masks of the last timed render, or None."""
     import numpy as np
 
     from gen3c_b200 import warp
@@ -234,17 +253,21 @@ def bench_path_r(torch, dev, peaks, steps: int, warmup: int, cpu_baseline: bool)
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
         for i in range(n):
-            fn(i)
+            out = fn(i)
         e.record()
         torch.cuda.synchronize()
-        return s.elapsed_time(e) / n
+        return s.elapsed_time(e) / n, out
 
     for i in range(max(3, warmup)):
         resident(i)
-    n = max(steps, 10)
-    ms = timed(resident, n)
+    n = steps
+    ms, (pix, msk) = timed(resident, n)
+    if outputs is not None:
+        outputs["path_r_pixels_sample"] = seeded_sample(torch, pix)
+        outputs["path_r_masks_sample"] = seeded_sample(torch, msk)
+    del pix, msk
     e2e(0)
-    ms_e2e = timed(e2e, n)
+    ms_e2e, _ = timed(e2e, n)
     px = R_FRAMES * R_H * R_W
     gbs = px * R_BYTES_PER_PX / (ms * 1e-3) / 1e9
     h2d = sum(t.numel() * t.element_size() for t in (depth_h, img_h, K_h, eye_h, w2cs_h, Ks_h))
@@ -492,13 +515,13 @@ def run_ours(args):
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
         for i in range(steps):
-            fn(i)
+            out = fn(i)
         e.record()
         barrier()
         ms = torch.tensor([s.elapsed_time(e)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms) / steps
+        return float(ms) / steps, out
 
     for i in range(max(3, args.warmup)):
         step_resident(i)
@@ -508,7 +531,9 @@ def run_ours(args):
     clocks.start()
     # -- timed region 1: inputs resident in HBM, profiling events on (per-category device time)
     _lib.check(lib.g3c_dit_profile(net._engine(), 1), "g3c_dit_profile")
-    ms_resident = timed(step_resident, args.steps)
+    ms_resident, x_next = timed(step_resident, args.steps)
+    outputs = {"x_next": x_next.float().cpu()} if args.dump_outputs else None
+    del x_next
     cat_ms = (C.c_float * 6)()
     cat_n = (C.c_int * 6)()
     _lib.check(lib.g3c_dit_profile_read(net._engine(), cat_ms, cat_n, 6), "g3c_dit_profile_read")
@@ -517,7 +542,7 @@ def run_ours(args):
     _lib.check(lib.g3c_dit_profile(net._engine(), 0), "g3c_dit_profile")
     # -- timed region 2: same step through the public API with pinned host buffers (H2D + D2H inside)
     step_e2e(0)
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     clk = clocks.finish()
     if rank != 0:
         if world > 1:
@@ -586,9 +611,11 @@ def run_ours(args):
         del devt
         torch.cuda.empty_cache()
         try:
-            line["path_r"] = bench_path_r(torch, dev, peaks, args.steps, args.warmup, not args.no_cpu_baseline)
+            line["path_r"] = bench_path_r(torch, dev, peaks, args.steps, args.warmup, not args.no_cpu_baseline, outputs)
         except Exception as ex:  # noqa: BLE001 - the second leg must never cost the headline line
             line["path_r"] = {"error": repr(ex)[:300]}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if world > 1:
         net._teardown_barrier()
@@ -633,7 +660,14 @@ def main():
                          "inside each half; cp = context parallel over all ranks (the reference's layout)")
     ap.add_argument("--cp-mode", default=None, choices=[None, "p2p", "nccl"],
                     help="context-parallel K/V exchange: p2p = fused projection -> peer-memory all-gather (default), nccl = ncclAllGather")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): the "
+                         "denoise step's x_(t-1) and a seeded sample of the Path R render")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl ours and --gpus 1")
     if args.impl == "reference":
         run_reference(args)
     else:

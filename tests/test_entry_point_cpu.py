@@ -5,7 +5,9 @@ import os
 import pytest
 import torch
 
-# option strings of cosmos_predict1/diffusion/inference/gen3c_single_image.py:35-99 + inference_utils.py:53-171
+# option strings of cosmos_predict1/diffusion/inference/gen3c_single_image.py:35-99 + inference_utils.py:53-171, stored
+# here so that the check needs no copy of the reference (its video-input options --input_image_or_video_path and
+# --num_input_frames are not taken by this entry point)
 REFERENCE_OPTIONS = [
     "--checkpoint_dir", "--tokenizer_dir", "--video_save_name", "--video_save_folder", "--prompt", "--batch_input_path",
     "--negative_prompt", "--num_steps", "--guidance", "--num_video_frames", "--height", "--width", "--fps", "--seed",
@@ -28,13 +30,6 @@ def test_command_line_surface_matches_reference():
     with pytest.raises(AssertionError):
         m.validate_args(p.parse_args(["--num_video_frames", "100"]))
     m.validate_args(p.parse_args(["--num_video_frames", "361"]))
-    ref = "/root/reference/cosmos_predict1/diffusion/inference/gen3c_single_image.py"
-    if os.path.exists(ref):  # in the build container: every option the reference declares is declared here
-        import re
-
-        txt = open(ref).read() + open("/root/reference/cosmos_predict1/diffusion/inference/inference_utils.py").read()
-        declared = set(re.findall(r'"(--[a-z_]+)"', txt))
-        assert declared - {"--input_image_or_video_path", "--num_input_frames"} <= have, declared - have
 
 
 def test_non_strict_load_reports_shapes_and_skips_te_state():
